@@ -224,6 +224,36 @@ def build_workload(spec, B, rank, pkg):
     return model, labels, loss_of
 
 
+OUTPUT_NAMES = {"asr": ("phoneme_loss", "word_loss", "phoneme_acc", "word_acc")}     # PretrainedModel.forward; Model.forward: loss, acc
+DUMP_LIMIT = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, kind, out, model, opt):
+    """What the last train step computed: the model's outputs, the gradients of the loss and Adam's first and second moments
+    after its update, each as out_dir/<out|grad|adam_m|adam_v>.<name>.npy in float32 or float64.  When dumping, every step
+    starts from the same weights (see `step` in main), so with the same arguments these agree from run to run up to the
+    rounding of the kernels' atomic gradient sums (<= 2e-6 of each tensor's largest element, measured on a B200 at 1000 W,
+    configs 3 and 4).  A gradient that is exactly zero in exact arithmetic holds only that rounding (config 5: the attention
+    key bias, to which the softmax is invariant), so compare it with an absolute tolerance.  The updated weights are not written: Adam divides each moment by its own magnitude + 1e-8, which turns
+    that rounding of near-zero gradients into weight differences of up to lr."""
+    import numpy as np
+    arrays = {"out." + n: t for n, t in zip(OUTPUT_NAMES.get(kind, ("loss", "acc")), out)}
+    for n, p in model.named_parameters():
+        if p.grad is not None:
+            arrays["grad." + n] = p.grad
+        st = opt.state.get(p, {})
+        if "exp_avg" in st:
+            arrays["adam_m." + n], arrays["adam_v." + n] = st["exp_avg"], st["exp_avg_sq"]
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes, more than the %d allowed" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -239,7 +269,12 @@ def main():
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip the reference-structured port on this GPU (cuDNN), N=1 only")
     ap.add_argument("--sampler-probe", action="store_true", help="developer: time the step under several clock-sampler settings (stderr)")
     ap.add_argument("--eval-dropout", action="store_true", help="disable dropout (debug)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed (model "
+                    "outputs, gradients, Adam moments) to DIR/<name>.npy, for comparing two builds output for output; every step "
+                    "then starts from the initial weights, which makes the results reproducible and the steps slower")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -279,11 +314,23 @@ def main():
     ys_dev = [tuple(y.cuda(non_blocking=True) for y in ys) for ys in ys_host]
     h2d_bytes = xs_host[0].numel() * 4 + sum(y.numel() * y.element_size() for y in ys_host[0])
 
+    last = {}                                                # outputs of the most recent step, for --dump-outputs
+    # With --dump-outputs every step trains from the initial weights.  The kernels sum gradients with atomics (last-bit order
+    # effects) and Adam amplifies those across steps into a different trajectory on every run; from fixed weights, batch and
+    # dropout seeds a step computes the same result each run.  The restore adds ~0.17 ms to a config-3 step (B200, 1000 W), so
+    # the times of a dumping run are not comparable with those of a plain one.
+    init_weights = [p.detach().clone() for p in params] if args.dump_outputs else None
+
     def step(x, ys):
-        loss = loss_of(model(x, *ys))
+        if init_weights is not None:
+            with torch.no_grad():
+                torch._foreach_copy_(params, init_weights)
+        out = model(x, *ys)
+        loss = loss_of(out)
         opt.zero_grad()
         loss.backward()
         opt.step()                                           # pre-step hook = the single gradient all-reduce
+        last["out"] = out
         return loss
 
     def barrier():
@@ -332,6 +379,8 @@ def main():
         ms_dev = timed(args.steps, host=None)
     launches = pkg._lib.stats["calls"] - calls0
     clk.stop()
+    if args.dump_outputs and rank == 0:                      # before any later step overwrites what the timed run left
+        dump_outputs(args.dump_outputs, kind, last["out"], model, opt)
     if args.sampler_probe and rank == 0:                     # developer: how much does the clock sampler perturb the timed region?
         for name, kw in [("none", None), ("25 ms full query", {}), ("25 ms, clocks + reasons only", {"query": ClockSampler.Q.replace("power.draw,", "")}),
                          ("100 ms full query", {"interval_ms": 100}), ("200 ms full query", {"interval_ms": 200}), ("none", None)]:
